@@ -18,6 +18,10 @@ One step = one pass of the hot path: K1 vectorise -> K2 top-n cosine product -> 
                (SURVEY.md §8d) are reported beside it as `algorithmic`
   parity       ALL pairs of the step's result against the CPU port's whole-job result (N=1)
   cpu_baseline the CPU port's measured whole job on this box's usable cores (N=1)
+
+--dump-outputs DIR writes the match list of the last timed step as .npy files (see dump_outputs) so that two builds
+can be compared output for output; the input corpus depends on --rows alone.  The benchmark writes nothing into the
+source tree (it may be read-only): the CPU whole-job cache lives in the system temp directory.
 """
 import argparse
 import atexit
@@ -179,6 +183,37 @@ def triples_digest(r, c, s):
     return h.hexdigest()[:32]
 
 
+DUMP_BYTES = 64_000_000
+DUMP_SAMPLE_ROWS = 1 << 18
+
+
+def dump_outputs(out_dir, triples, n, seed=0):
+    """Write a match list (row, col, score triples) as float64 .npy files under `out_dir`:
+
+      pairs_per_row  (n,)  pairs of every row
+      sample_rows    sorted rows of a fixed sample: the first DUMP_SAMPLE_ROWS of a permutation seeded by `seed`,
+                     fewer only if their pairs would take the files past DUMP_BYTES
+      row, col, score  every pair of the sampled rows, sorted by (row, col)
+
+    Row and column indices are exact in float64."""
+    r = np.asarray(triples[0]).astype(np.int64)
+    c = np.asarray(triples[1]).astype(np.int64)
+    s = np.asarray(triples[2]).astype(np.float64)
+    counts = np.bincount(r, minlength=n)
+    order = np.random.default_rng(seed).permutation(n)[:DUMP_SAMPLE_ROWS]
+    budget = DUMP_BYTES // 8 - n - 5 * 16             # float64 elements left (pairs_per_row, .npy headers)
+    cost = np.cumsum(1 + 3 * counts[order])           # one sample_rows entry + row, col, score per pair
+    rows = np.sort(order[:int(np.searchsorted(cost, budget, side="right"))])
+    sel = np.zeros(n, dtype=bool)
+    sel[rows] = True
+    sel = sel[r]
+    o = np.lexsort((c[sel], r[sel]))
+    arrays = {"pairs_per_row": counts, "sample_rows": rows, "row": r[sel][o], "col": c[sel][o], "score": s[sel][o]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 # ----------------------------------------------------------------------------- B200 arm
 def main():
     ap = argparse.ArgumentParser()
@@ -191,7 +226,14 @@ def main():
     ap.add_argument("--no-aux", action="store_true", help="multi-GPU: skip the two-Series sharded-K1 run")
     ap.add_argument("--aux-master", type=int, default=2_000_000)
     ap.add_argument("--aux-duplicates", type=int, default=400_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the match list of the last timed step under DIR as .npy files (B200 arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    sys.dont_write_bytecode = True          # no __pycache__ in the source tree for the project modules imported below
 
     if os.environ.get("NCCL_DEBUG", "").upper() == "VERSION":
         os.environ["NCCL_DEBUG"] = "WARN"           # keep stdout to the one JSON line
@@ -470,6 +512,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return 0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, final_triples, n)
 
     # ---- CPU port on this box: measured whole job -> cpu_baseline + parity of ALL pairs (N=1 only) ----
     cpu_baseline = parity = None
@@ -485,7 +529,7 @@ def main():
             job = C.whole_job(names, cores)
         parity = C.compare(job, pre_triples, final_triples)
         parity["cpu_job"] = "measured by this process" if not job.get("from_cache") else \
-            "measured by `bench.py --impl reference` on this box earlier in this boot (oracle/_cache)"
+            "measured by `bench.py --impl reference` on this box earlier in this boot (bench_cpu.CACHE_DIR)"
         cpu_baseline = {"value": job["pairs"] / job["wall_s"], "unit": UNIT, "cores": job["threads"], "kind": "port",
                         "sample": "the WHOLE job, measured once on this box (%d names, n_blocks=%s, %d OpenMP threads; "
                                   "os.cpu_count() = %s, usable = %d): %.1f s, phases %s"

@@ -1,6 +1,9 @@
 """not-gpu: the C-ABI library loads and exports every symbol include/sg_b200.h declares (no compute calls)."""
 import os
 import re
+import subprocess
+import sys
+import textwrap
 
 from string_grouper_b200 import _lib
 
@@ -37,12 +40,25 @@ def test_no_product_module_imports_the_oracle():
             assert "oracle" not in re.sub(r'""".*?"""', "", src, flags=re.S).replace("# oracle", ""), fn
 
 
-def test_missing_device_fails_loudly():
+MISSING_DEVICE = textwrap.dedent('''
+    import sys
+    sys.path.insert(0, %r)
     import pandas as pd
-    import pytest
     import torch
-    if torch.cuda.is_available():
-        pytest.skip("CUDA present")
+    assert not torch.cuda.is_available()
     import string_grouper_b200 as api
-    with pytest.raises(_lib.SgB200Error):
+    from string_grouper_b200 import _lib
+    try:
         api.match_strings(pd.Series(["foo inc", "foo inc."]))
+    except _lib.SgB200Error:
+        sys.exit(0)
+    sys.exit("no SgB200Error without a CUDA device")
+''')
+
+
+def test_missing_device_fails_loudly():
+    # a child process that sees no device, so that the check also runs on a machine with GPUs
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-c", MISSING_DEVICE % ROOT], env=env, capture_output=True, text=True,
+                       timeout=600)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]

@@ -1,25 +1,23 @@
 """not-gpu: pins the CPU oracle (oracle/) against the answers of the UNMODIFIED reference.
 
-  * tests/golden/synthetic.npz was produced by /root/reference + the oracle stand-in (oracle/make_golden.py);
+  * tests/golden/synthetic.npz was produced by the reference + the oracle stand-in (oracle/make_golden.py);
     the oracle's own restatement of fit() (oracle/pipeline.py) must reproduce it exactly;
-  * when /root/reference is present (the build container) the reference's own unittest suite is run
-    against the stand-in: every hot-path test must pass (the 4 add_match tests fail on pandas 3's
-    removed Series._append, off the hot path — SURVEY.md §0 fact 4).
+  * tests/golden/standin_calls.npz holds every distinct call the reference's own unittest suite made into the
+    stand-in, with the stand-in's answers, recorded while that suite passed (oracle/record_standin_calls.py): every
+    hot-path test passed (the add_match tests fail on pandas 3's removed Series._append, off the hot path —
+    SURVEY.md §0 fact 4).  Replaying the calls must give the same answers bit for bit.
 """
+import json
 import os
-import subprocess
-import sys
 
 import numpy as np
-import pytest
-from scipy.sparse import csr_matrix
+from scipy.sparse import csc_matrix, csr_matrix
 
 from oracle import pipeline as P
 from oracle.sdt import sp_matmul_topn, zip_sp_matmul_topn
 from synth_corpus import make_names
 
 GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "synthetic.npz"), allow_pickle=True)
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_pipeline_restatement_reproduces_reference_self_match():
@@ -80,16 +78,32 @@ def test_block_invariance_of_the_oracle():
         assert abs(base - other).max() < 1e-12 or (base != other).nnz <= 4   # top-n ties may swap
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/string_grouper"), reason="reference tree not present")
 def test_reference_own_suite_passes_with_the_oracle_standin():
-    env = dict(os.environ)
-    env["PYTHONPATH"] = os.pathsep.join([os.path.join(ROOT, "oracle", "standin"), "/root/reference"])
-    r = subprocess.run([sys.executable, "-m", "pytest", "/root/reference/string_grouper/test/test_string_grouper.py",
-                        "-q", "-p", "no:cacheprovider", "--deselect",
-                        "string_grouper/test/test_string_grouper.py::StringGrouperTest::test_add_match_single_occurence"],
-                       capture_output=True, text=True, env=env, cwd="/tmp")
-    tail = r.stdout.strip().splitlines()[-1]
-    failed = [ln for ln in r.stdout.splitlines() if ln.startswith("FAILED")]
-    # only the pandas-3 `Series._append` removals may fail (add_match, off the hot path)
-    assert all("add_match" in ln or "prior_matches" in ln for ln in failed), r.stdout[-2000:]
-    assert "passed" in tail and int(tail.split(" passed")[0].split()[-1]) >= 49, tail
+    z = np.load(os.path.join(os.path.dirname(__file__), "golden", "standin_calls.npz"), allow_pickle=False)
+    meta = json.loads(str(z["meta"]))
+    values, ints = z["values"], z["ints"]
+    suite = meta["suite"]
+    # only the pandas-3 `Series._append` removals failed (add_match, off the hot path)
+    assert all("add_match" in t or "prior_matches" in t for t in suite["failed"]), suite
+    assert suite["passed"] >= 49, suite
+
+    def load(rec):
+        v0, nv = rec["values"]
+        i0, ni = rec["indices"]
+        p0, npp = rec["indptr"]
+        parts = (values[v0:v0 + nv].astype(rec["dtype"]), ints[i0:i0 + ni].astype(rec["index_dtype"]),
+                 ints[p0:p0 + npp].astype(rec["index_dtype"]))
+        return (csr_matrix if rec["format"] == "csr" else csc_matrix)(parts, shape=tuple(rec["shape"]))
+
+    assert len(meta["calls"]) > 100 and {c["fn"] for c in meta["calls"]} == {"sp_matmul_topn", "zip_sp_matmul_topn"}
+    for i, c in enumerate(meta["calls"]):
+        if c["fn"] == "sp_matmul_topn":
+            got = sp_matmul_topn(load(c["A"]), load(c["B"]), *c["args"], **c["kwargs"])
+        else:
+            got = zip_sp_matmul_topn(top_n=c["top_n"], C_mats=[load(m) for m in c["C_mats"]])
+        want = load(c["out"])
+        label = "call %d (%s)" % (i, c["fn"])
+        assert got.format == "csr" and got.shape == want.shape and got.dtype == want.dtype, label
+        assert got.indices.dtype == want.indices.dtype, label
+        assert np.array_equal(got.indptr, want.indptr) and np.array_equal(got.indices, want.indices), label
+        assert np.array_equal(got.data, want.data), label
