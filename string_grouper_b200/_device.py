@@ -4,7 +4,7 @@ PyTorch is used for device memory, streams and (in _dist.py) torch.distributed
 only; every kernel on the hot path lives in csrc/*.cu behind the C ABI.
 """
 import ctypes
-import os
+from typing import NamedTuple
 
 import numpy as np
 
@@ -19,30 +19,28 @@ LAUNCH_COUNTS = {"postings": 0, "candidates": 0, "rescore": 0, "select": 0, "sym
 
 TRANSFER_BYTES = {"d2h": 0, "h2d": 0}      # bytes moved by the bulk copies (bench.py e2e accounting)
 
-DEFAULT_TILE_W = int(os.environ.get("SG_B200_TILE_W", "0"))         # 0: 256 (u16) columns per tile, 128 for large right matrices
-DEFAULT_WARPS = int(os.environ.get("SG_B200_WARPS", "8"))           # 8 warps x 5 CTAs at 48 registers (no spills)
-GROUP_BYTES = int(os.environ.get("SG_B200_GROUP_MB", "12")) << 20   # posting bytes one column-tile group may hold
+DEFAULT_WARPS = 8        # 8 warps x 5 CTAs at 48 registers (no spills)
+GROUP_BYTES = 12 << 20   # posting bytes one column-tile group may hold
 CAND_MARGIN = 1.5e-3   # candidates: fp16 posting weights (<= 4.9e-4) + fp32 accumulation; all are re-scored exactly
 U16_MARGIN_PER_FEATURE = 2e-5   # 1/32768 fixed-point accumulator tile: one rounding of <= 2^-16 per added product
 # Exact threshold pruning (csrc/sg_prune.cu): the most expensive heavy features of a left row are skipped while
 # their norm times the largest right-row norm stays below PRUNE_FRAC * min_similarity.  0 switches it off.
-PRUNE_FRAC = float(os.environ.get("SG_B200_PRUNE", "0.9"))
-ACC_DTYPE = os.environ.get("SG_B200_ACC", "u16")                    # accumulator tile: u16 | f32
-MAX_CAND_DENSITY = float(os.environ.get("SG_B200_MAX_CAND_DENSITY", "1.5e-3"))   # candidates per (row, column) pair
-MAX_BUCKETS = int(os.environ.get("SG_B200_MAX_BUCKETS", str(400_000_000)))       # directory entries (22 B each)
-CAND_CHUNK = int(os.environ.get("SG_B200_CAND_CHUNK", str(1 << 28)))            # candidates per chunk of left rows
+PRUNE_FRAC = 0.9
+ACC_DTYPE = "u16"               # accumulator tile: u16 | f32
+MAX_CAND_DENSITY = 1.5e-3       # candidates per (row, column) pair
+MAX_BUCKETS = 400_000_000       # directory entries (22 B each)
+CAND_CHUNK = 1 << 28            # candidates per chunk of left rows
 # up to this many (left row, right row) pairs the candidates kernel is launched without a sizing pass (see cossim_topn)
-OPTIMISTIC_PAIRS = float(os.environ.get("SG_B200_OPTIMISTIC_PAIRS", "5e11"))
-REFINE = os.environ.get("SG_B200_REFINE", "1") != "0"      # grouped per-candidate bound before the exact re-score
+OPTIMISTIC_PAIRS = 5e11
+REFINE = True                   # grouped per-candidate bound before the exact re-score
 # K2 formulation: "row" (the default) = one warp per left row over L2-resident posting buckets (csrc/sg_cossim.cu; also
 # the general path: negative values, norms above 1, near-zero thresholds); "tiles" = right tiles staged through TMA into
 # shared memory (csrc/sg_tiles.cu), for L2-normalised non-negative operands.  Measured on B200 at 663k rows the row kernel
 # is the faster one (DESIGN.md §4: both are bound by instruction issue at ~340 warp instructions per (row, tile) pair).
-K2_KERNEL = os.environ.get("SG_B200_KERNEL", "row").lower()
+K2_KERNEL = "row"
 TILE_MARGIN = 2e-5               # fp32 arithmetic of thresholds / norms and the f64 -> f32 copy of the values
 TILE_MARGIN_PER_FEATURE = 3.1e-5  # a_q * w_q / 2^30 vs a * w: both weights rounded to nearest 2^-15 (<= 2^-15 + 2^-32)
-TILE_WARPS = int(os.environ.get("SG_B200_TILE_WARPS", "8"))
-SELECT_MODE = os.environ.get("SG_B200_SELECT", "rows").lower()      # "rows" (per-row ranking) | "sort" (global sorts)
+SELECT_MODE = "rows"            # "rows" (per-row ranking) | "sort" (global sorts)
 
 
 def torch():
@@ -273,10 +271,22 @@ def right_order(B):
     return B._order
 
 
+def _tile_bounds(B, perm, tile_w):
+    """Largest heavy norm of B's rows per column tile of `tile_w` rows of the processing order `perm`
+    (sg_tile_bounds): the per-tile pruning bound."""
+    t = torch()
+    L = _lib.load()
+    bound = t.zeros(int(L.sg_num_tiles_padded(B.shape[0], tile_w)), dtype=t.float32, device=B.device)
+    _lib.check(L.sg_tile_bounds(B.shape[0], _ptr(perm), _ptr(B._heavy_norm), tile_w, _ptr(bound), _stream()))
+    LAUNCH_COUNTS["prune"] += 1
+    return bound
+
+
 def right_tiles(B):
     """Tile blobs of the tile-centric K2 (csrc/sg_tiles.cu), cached on B: per 256-row tile of the processing order
     the postings sorted by feature, the bitmap directory and the bucket offsets as one blob (what the candidates
-    kernel stages through TMA), the fp16 block maxima of every (feature, tile) and the per-tile pruning bound."""
+    kernel stages through TMA), the fp16 block maxima of every (feature, tile), the per-tile pruning bound and the
+    bytes the kernel stages per tile (read back once)."""
     t = require_cuda()
     L = _lib.load()
     hrank, perm, rank = right_order(B)
@@ -296,11 +306,9 @@ def right_tiles(B):
                                     _ptr(rank), B.base, 1.0 / max(B.norm_bound, 1.0), _ptr(desc), _ptr(blob), cap,
                                     _ptr(maxw), _ptr(maxima), _ptr(ws), ws_bytes, _stream()))
         LAUNCH_COUNTS["tiles"] += 4
-        bound = t.zeros(Tp, dtype=t.float32, device=B.device)
-        _lib.check(L.sg_tile_bounds(n_rows, _ptr(perm), _ptr(B._heavy_norm), W, _ptr(bound), _stream()))
-        LAUNCH_COUNTS["prune"] += 1
+        bound = _tile_bounds(B, perm, W)
         B._tiles = {"desc": desc, "blob": blob, "maxw": maxw, "bound": bound, "maxima": maxima, "T": T, "W": W,
-                    "stage_bytes": None}
+                    "stage_bytes": int(maxima[0].item())}
     return B._tiles
 
 
@@ -328,9 +336,7 @@ def right_side(B, tile_w):
                                        _ptr(bucket_dir), _ptr(bucket_maxw), _ptr(post),
                                        _ptr(ws), ws_bytes, _stream()))
         LAUNCH_COUNTS["postings"] += 4
-        bound = t.zeros(Tp, dtype=t.float32, device=B.device)
-        _lib.check(L.sg_tile_bounds(n_rows, _ptr(perm), _ptr(B._heavy_norm), tile_w, _ptr(bound), _stream()))
-        LAUNCH_COUNTS["prune"] += 1
+        bound = _tile_bounds(B, perm, tile_w)
         B._postings2[tile_w] = (bucket_dir, bucket_maxw, post, T, bound)     # bucket_ptr is only needed for the build
     return (hrank, perm, rank) + B._postings2[tile_w]
 
@@ -412,11 +418,106 @@ def pick_tile(n_right, tile_w=None, warps=None, acc_bytes=4, n_left=None):
     # (the finer directory costs ~0.6 ms more to build: not worth it for a small block of left rows, e.g. one of 8 shards)
     many_left = n_left is None or int(n_left) >= 150_000
     auto_w = 128 if (acc_bytes == 4 or (int(n_right) >= 400_000 and many_left)) else 256
-    tile_w = int(tile_w or DEFAULT_TILE_W) or auto_w
+    tile_w = int(tile_w or auto_w)
     q = 256 // acc_bytes                               # tile bytes must be a multiple of 256
     need = ((max(int(n_right), 1) + q - 1) // q) * q
     tile_w = max(q, min(tile_w, 32768) // q * q)
     return min(tile_w, need), warps
+
+
+def k2_accumulator(acc, threshold, scale, nonneg):
+    """(accumulator tile, candidate threshold) of K2: the tile the caller asked for (default ACC_DTYPE) and
+    threshold - CAND_MARGIN * max(scale, 1) clamped at 0.  `scale` bounds every score (the product of the operands'
+    largest row norms); `nonneg`: no negative stored value in either operand."""
+    thr_c = max(float(threshold) - CAND_MARGIN * max(scale, 1.0), 0.0)
+    acc = (acc or ACC_DTYPE).lower()
+    if acc not in ("u16", "f32"):
+        raise ValueError("accumulator dtype must be 'u16' or 'f32', got %r" % (acc,))
+    # fixed-point accumulator tiles need non-negative weights and scores below 2 (K1's L2-normalised rows); also
+    # near-zero thresholds take fp32: a tiny positive score must not round to a fixed-point zero
+    if not (nonneg and scale <= 1.0 + 1e-6) or thr_c < 0.05:
+        acc = "f32"
+    return acc, thr_c
+
+
+class K2Plan(NamedTuple):
+    """What cossim_topn decides before its first candidates launch (plan_k2)."""
+    kernel: str              # "row" (csrc/sg_cossim.cu) | "tiles" (csrc/sg_tiles.cu)
+    acc: str                 # accumulator tile: "u16" | "f32"
+    margin: float            # score error of the candidate traversal ...
+    margin_pf: float         # ... plus this much per kept feature of the left row (fixed-point products)
+    thr_c: float             # candidate threshold
+    tile_w: int              # columns per tile
+    warps: int               # warps per CTA
+    tiles_per_group: int     # column tiles per work group of the row kernel (0: tile formulation)
+    refine: bool             # candidates carry their partial score; sg_rescore_refined re-tests them first
+    levels: tuple            # pruning levels, in the order they are tried
+    whole_range: bool        # one launch over every row at levels[0] before any sizing pass
+    sample_stride: int       # every stride-th row of the processing order sizes the buffers (None: no sample)
+    cand_limit: float        # a lower pruning level is tried above this many candidates (MAX_CAND_DENSITY)
+
+
+def plan_k2(n_rows, n_right, n_cols, nnz_right, threshold, scale=1.0, nonneg=True, kernel=None, acc=None, prune=None,
+            tile_w=None, warps=None, tile_fit=None):
+    """K2's decisions for `n_rows` left rows against a right matrix of n_right x n_cols with nnz_right stored values;
+    the arguments after `nonneg` are those of cossim_topn.
+
+    tile_fit: (tile width, shared memory the tile kernel needs at 8 warps, the device's opt-in shared memory per
+    block) of the right matrix's tile blobs (right_tiles); cossim_topn builds them only when the tile formulation is
+    asked for, the fixed-point accumulator applies and the bitmap directory holds every feature.  Without it, or
+    when the stage does not fit shared memory, the row kernel runs."""
+    acc, thr_c = k2_accumulator(acc, threshold, scale, nonneg)
+    kernel = (kernel or K2_KERNEL).lower()
+    if kernel not in ("tiles", "row"):
+        raise ValueError("kernel must be 'tiles' or 'row', got %r" % (kernel,))
+    if kernel == "tiles" and acc == "u16" and tile_fit is not None and tile_fit[1] <= tile_fit[2]:
+        margin, margin_pf = TILE_MARGIN * max(scale, 1.0), TILE_MARGIN_PER_FEATURE
+        tile_w, warps, tiles_per_group = tile_fit[0], 8, 0
+    else:
+        kernel, margin = "row", CAND_MARGIN * max(scale, 1.0)
+        margin_pf = U16_MARGIN_PER_FEATURE if acc == "u16" else 0.0
+        tile_w, warps = pick_tile(n_right, tile_w, warps, 2 if acc == "u16" else 4, n_left=n_rows)
+        # the bucket directory holds one entry per (feature, tile): widen the tiles until it stays below MAX_BUCKETS
+        while (-(-n_right // tile_w)) * (n_cols + 1) > MAX_BUCKETS and tile_w < 32768:
+            tile_w *= 2
+        n_tiles = -(-n_right // tile_w)
+        # column tiles per work group (a multiple of 64): the group's posting buckets should stay L2-resident
+        tiles_per_group = max(64, int(GROUP_BYTES // max(4 * nnz_right / n_tiles, 1)) // 64 * 64)
+    # when the caller left the pruning level open it may be lowered (see _size_candidates)
+    level = PRUNE_FRAC if prune is None else float(prune)
+    levels = (level,)
+    if prune is None and level > 0.0 and thr_c > 0.0:
+        levels = (level, 0.75 * level, 0.5 * level, 0.25 * level, 0.0)
+    return K2Plan(kernel=kernel, acc=acc, margin=margin, margin_pf=margin_pf, thr_c=thr_c, tile_w=tile_w, warps=warps,
+                  tiles_per_group=tiles_per_group, refine=REFINE and kernel == "row" and acc == "u16", levels=levels,
+                  whole_range=float(n_rows) * float(n_right) <= OPTIMISTIC_PAIRS,
+                  sample_stride=max(64, n_rows // 8192) if n_rows >= 65536 else None,
+                  cand_limit=MAX_CAND_DENSITY * n_rows * n_right)
+
+
+def row_chunks(n_rows, est):
+    """(chunks, rows per chunk): slices of the processing order whose candidates, `est` for all rows with 30 %
+    headroom, fit CAND_CHUNK entries; one chunk without an estimate."""
+    n_chunks = 1 if est is None else max(1, -(-int(1.3 * est) // CAND_CHUNK))
+    return n_chunks, -(-n_rows // n_chunks)
+
+
+def chunk_capacity(n_rows, rows, est):
+    """Candidate buffer entries for a chunk of `rows` of the `n_rows` left rows, `est` candidates expected for all of
+    them.  Without an estimate a guess: clusters of identical names make the candidates much more than top_n per row
+    (37 M for the 663k benchmark corpus); a chunk that overflows is launched again with the exact count."""
+    if est is None:
+        return min(96 * n_rows + (1 << 22), 1 << 30)
+    return min(int(1.3 * est * rows / n_rows) + (1 << 22), 1 << 31)
+
+
+def select_mode(top_n, max_row_cnt, rows_cap):
+    """"rows": survivors bucketed by row, every row ranked on its own (warp shuffle network, or one CTA in shared
+    memory for up to `rows_cap` = sg_topn_rows_cap() survivors, longer rows in pieces while top_n <= rows_cap / 2);
+    "sort": three global radix sorts.  `max_row_cnt`: survivors of the longest row."""
+    if SELECT_MODE != "sort" and (top_n <= 32 or max_row_cnt <= rows_cap or top_n <= rows_cap // 2):
+        return "rows"
+    return "sort"
 
 
 def feature_df(B):
@@ -462,7 +563,6 @@ def cossim_topn(A, B, top_n, threshold, row_begin=0, row_end=None, tile_w=None, 
     (string_grouper.py:734-750).  Returns DeviceMatches with absolute row ids.
     """
     t = require_cuda()
-    L = _lib.load()
     if A.shape[1] != B.shape[1]:
         raise ValueError("dimension mismatch: left has %d features, right has %d" % (A.shape[1], B.shape[1]))
     if A.dtype != B.dtype:
@@ -471,312 +571,329 @@ def cossim_topn(A, B, top_n, threshold, row_begin=0, row_end=None, tile_w=None, 
     row_end = n_left if row_end is None else int(row_end)
     row_begin = int(row_begin)
     n_rows = max(row_end - row_begin, 0)
-    dev = A.device
     top_n = int(min(int(top_n), n_right))
-    dt = _lib.SG_DTYPE_F32 if A.dtype == np.float32 else _lib.SG_DTYPE_F64
-    shape = (n_left, n_right)
     if n_rows == 0 or n_right == 0 or top_n <= 0 or A.nnz == 0 or B.nnz == 0:
-        z32 = _empty(1, t.int32, dev)
-        return DeviceMatches(shape, z32, z32, _empty(1, t.float64, dev), 0, 0)
+        z32 = _empty(1, t.int32, A.device)
+        return DeviceMatches((n_left, n_right), z32, z32, _empty(1, t.float64, A.device), 0, 0)
 
     mark(stats, "k2_start")
-    scale = A.norm_bound * B.norm_bound
-    margin = CAND_MARGIN * max(scale, 1.0)
-    thr_c = max(float(threshold) - margin, 0.0)
-    # fixed-point accumulator tiles need non-negative weights and scores below 2 (K1's L2-normalised rows)
-    acc = (acc or ACC_DTYPE).lower()
-    if acc not in ("u16", "f32"):
-        raise ValueError("accumulator dtype must be 'u16' or 'f32', got %r" % (acc,))
-    if not (A.nonneg and B.nonneg and scale <= 1.0 + 1e-6) or thr_c < 0.05:
-        acc = "f32"      # also near-zero thresholds: a tiny positive score must not round to a fixed-point zero
-    acc_code = _lib.SG_ACC_U16 if acc == "u16" else _lib.SG_ACC_F32
-    margin_pf = U16_MARGIN_PER_FEATURE if acc == "u16" else 0.0
-    # tile-centric kernel: fixed-point products need what the u16 tiles need; the bitmap directory bounds the features
-    kernel = (kernel or K2_KERNEL).lower()
-    if kernel not in ("tiles", "row"):
-        raise ValueError("kernel must be 'tiles' or 'row', got %r" % (kernel,))
-    use_tiles = kernel == "tiles" and acc == "u16" and B.shape[1] <= int(L.sg_tiles_max_cols())
-    tiles = None
-    if use_tiles:
-        tiles = right_tiles(B)
-        if tiles["stage_bytes"] is None:
-            tiles["stage_bytes"] = int(tiles["maxima"][0].item())       # one read-back per right matrix
-        smem_optin = t.cuda.get_device_properties(dev).shared_memory_per_block_optin
-        tile_warps = next((w for w in (TILE_WARPS, 8) if w in (8, 16) and
-                           int(L.sg_tiles_smem_bytes(tiles["stage_bytes"], w)) <= smem_optin), None)
-        if tile_warps is None:
-            use_tiles, tiles = False, None          # a tile's index does not fit shared memory: row kernel
-    if use_tiles:
-        margin = TILE_MARGIN * max(scale, 1.0)
-        margin_pf = TILE_MARGIN_PER_FEATURE
-    prune_auto = prune is None          # the caller left the level open: it may be lowered, see below
-    prune = PRUNE_FRAC if prune is None else float(prune)
-    counters = t.zeros(4, dtype=t.int64, device=dev)       # [0] cand_count, [1] work queue
-    # candidate buffer: clusters of identical names make this much larger than top_n * rows (37 M for the
-    # 663k benchmark corpus); a second launch with the exact size happens only if this guess is too small
-    cap = int(os.environ.get("SG_B200_CAND_CAP", 0)) or min(96 * n_rows + (1 << 22), 1 << 30)
-    # both operands in the same processing order (quantised heavy norm, heavy-feature signature): neighbouring left
-    # rows stream the same buckets, and the rows of a column tile have similar heavy norms (tight per-tile bound)
-    if use_tiles:
-        hrank, perm_b, _ = right_order(B)
-        tile_w, warps, T, tile_bound = tiles["W"], tile_warps, tiles["T"], tiles["bound"]
-        tiles_per_group = 0
-        lpack = _empty(2 * A.d_indices.numel(), t.int32, dev)
-        mask_words = int(L.sg_tiles_mask_words(n_right))
-    else:
-        tile_w, warps = pick_tile(n_right, tile_w, warps, 2 if acc == "u16" else 4, n_left=n_rows)
-        # the bucket directory holds one entry per (feature, tile): widen the tiles until it stays below MAX_BUCKETS
-        while (-(-n_right // tile_w)) * (B.shape[1] + 1) > MAX_BUCKETS and tile_w < 32768:
-            tile_w *= 2
-        hrank, perm_b, _, bucket_dir, bucket_maxw, post, T, tile_bound = right_side(B, tile_w)
-        # column tiles per work group (a multiple of 64): the group's posting buckets should stay L2-resident
-        tiles_per_group = max(64, int(GROUP_BYTES // max(4 * B.nnz / T, 1)) // 64 * 64)
-    if A is B and row_begin == 0 and row_end == n_left:
-        perm_a = perm_b
-    else:
-        perm_a, _ = row_order(A, hrank, row_begin, row_end, want_rank=False)
+    plan = _plan(A, B, n_rows, threshold, kernel, acc, prune, tile_w, warps)
+    k = _K2Call(A, B, row_begin, row_end, threshold, plan)
     mark(stats, "right_side")
-    c_count = ctypes.c_void_p(counters.data_ptr())
-    c_queue = ctypes.c_void_p(counters.data_ptr() + 8)
-    c_walk = ctypes.c_void_p(counters.data_ptr() + 16)
-    dummy = _empty(1, t.int32, dev)
-    pruned = {}
+    survivors = _candidates_rescored(k, stats)
+    if stats is not None:
+        stats["tile_w"], stats["warps"], stats["n_tiles"] = plan.tile_w, plan.warps, k.n_tiles
+        stats["tiles_per_group"] = plan.tiles_per_group
+        if plan.kernel == "tiles":
+            stats["stage_bytes"] = k.tiles["stage_bytes"]
+    return _select(k, top_n, *survivors, stats)
 
-    def launch_tiles(perm, n, row_buf, col_buf, capacity):
-        """pack the pruned rows of `perm`, block-max filter -> survivor bits, tile kernel"""
-        l_idx, l_val, l_len, l_thr, l_xp, _ = pruned["arrays"]
+
+def _plan(A, B, n_rows, threshold, kernel, acc, prune, tile_w, warps):
+    """plan_k2 for one call.  The tile formulation's fit check needs its blobs: they are built here when it may run."""
+    t = torch()
+    L = _lib.load()
+    scale, nonneg = A.norm_bound * B.norm_bound, A.nonneg and B.nonneg
+    tile_fit = None
+    if ((kernel or K2_KERNEL).lower() == "tiles" and k2_accumulator(acc, threshold, scale, nonneg)[0] == "u16"
+            and B.shape[1] <= int(L.sg_tiles_max_cols())):
+        tiles = right_tiles(B)
+        tile_fit = (tiles["W"], int(L.sg_tiles_smem_bytes(tiles["stage_bytes"], 8)),
+                    t.cuda.get_device_properties(A.device).shared_memory_per_block_optin)
+    return plan_k2(n_rows, B.shape[0], B.shape[1], B.nnz, threshold, scale, nonneg, kernel=kernel, acc=acc,
+                   prune=prune, tile_w=tile_w, warps=warps, tile_fit=tile_fit)
+
+
+class _K2Call:
+    """Device arrays of one cossim_topn call: the right side in the plan's formulation (`tiles`, or the row kernel's
+    bucket directory, block maxima and postings), both operands' processing orders and the counters the kernels
+    report through ([0] candidates / survivors, [1] work queue / longest row, [2] pairs walked / refined candidates,
+    [3] postings walked)."""
+
+    def __init__(self, A, B, row_begin, row_end, threshold, plan):
+        t = torch()
+        self.A, self.B, self.plan, self.threshold = A, B, plan, float(threshold)
+        self.row_begin, self.row_end, self.n_rows = row_begin, row_end, row_end - row_begin
+        self.counters = t.zeros(4, dtype=t.int64, device=A.device)
+        # both operands in the same processing order (quantised heavy norm, heavy-feature signature): neighbouring left
+        # rows stream the same buckets, and the rows of a column tile have similar heavy norms (tight per-tile bound)
+        if plan.kernel == "tiles":
+            self.tiles = right_tiles(B)
+            self.hrank, self.perm_b, _ = right_order(B)
+            self.n_tiles, self.tile_bound = self.tiles["T"], self.tiles["bound"]
+            self.lpack = _empty(2 * A.d_indices.numel(), t.int32, A.device)
+        else:
+            (self.hrank, self.perm_b, _, self.bucket_dir, self.bucket_maxw, self.post, self.n_tiles,
+             self.tile_bound) = right_side(B, plan.tile_w)
+        if A is B and row_begin == 0 and row_end == A.shape[0]:
+            self.perm_a = self.perm_b
+        else:
+            self.perm_a, _ = row_order(A, self.hrank, row_begin, row_end, want_rank=False)
+
+    def counter(self, i):
+        return ctypes.c_void_p(self.counters.data_ptr() + 8 * i)
+
+
+def _prune(k, level):
+    """The call's left rows pruned at `level` (prune_left; the fixed-point tile always takes per-row thresholds: its
+    margin grows with the number of features added), or A's own arrays when neither applies."""
+    p = k.plan
+    if (level > 0.0 and p.thr_c > 0.0) or p.margin_pf > 0.0:
+        return prune_left(k.A, k.B, k.hrank, k.row_begin, k.row_end, k.threshold, p.margin, p.margin_pf,
+                          level if p.thr_c > 0.0 else 0.0)
+    return k.A.d_indices, k.A.d_val32, None, None, None, None
+
+
+def _launch_candidates(k, pruned, perm, n, row_buf, col_buf, capacity, partial_buf=None):
+    """Candidates of the left rows perm[:n] into (row_buf, col_buf, partial_buf)[:capacity]; counters[0] = their
+    number, which may exceed `capacity`."""
+    t = torch()
+    L = _lib.load()
+    A, B, p = k.A, k.B, k.plan
+    l_idx, l_val, l_len, l_thr, l_xp, _ = pruned
+    if p.kernel == "tiles":
+        # pack the pruned rows of `perm`, block-max filter -> survivor bits, tile kernel
         stride = (n + 31) // 32 * 32
-        rowinfo = _empty(4 * stride, t.int32, dev)
-        mask = _empty(mask_words * stride, t.int32, dev)
-        counters.zero_()
+        rowinfo = _empty(4 * stride, t.int32, A.device)
+        mask = _empty(int(L.sg_tiles_mask_words(B.shape[0])) * stride, t.int32, A.device)
+        k.counters.zero_()
         _lib.check(L.sg_tiles_pack_left(n, _ptr(perm), 0, _ptr(A.d_indptr), _ptr(l_len), _ptr(l_idx), _ptr(l_val),
-                                        _ptr(l_thr), _ptr(l_xp), max(B.norm_bound, 1.0), _ptr(lpack), _ptr(rowinfo),
-                                        _stream()))
-        _lib.check(L.sg_tiles_filter(n, _ptr(rowinfo), _ptr(lpack), _ptr(tiles["maxw"]), n_right, _ptr(tile_bound),
-                                     _ptr(mask), stride, _stream()))
-        _lib.check(L.sg_tiles_candidates(_ptr(perm), n, 0, _ptr(rowinfo), _ptr(lpack), _ptr(mask), stride,
-                                         _ptr(tiles["desc"]), _ptr(tiles["blob"]), n_right, B.shape[1],
-                                         _ptr(tile_bound), _ptr(perm_b), tiles["stage_bytes"], _ptr(row_buf),
-                                         _ptr(col_buf), capacity, c_count, c_queue, c_walk, warps, _stream()))
+                                        _ptr(l_thr), _ptr(l_xp), max(B.norm_bound, 1.0), _ptr(k.lpack),
+                                        _ptr(rowinfo), _stream()))
+        _lib.check(L.sg_tiles_filter(n, _ptr(rowinfo), _ptr(k.lpack), _ptr(k.tiles["maxw"]), B.shape[0],
+                                     _ptr(k.tile_bound), _ptr(mask), stride, _stream()))
+        _lib.check(L.sg_tiles_candidates(_ptr(perm), n, 0, _ptr(rowinfo), _ptr(k.lpack), _ptr(mask), stride,
+                                         _ptr(k.tiles["desc"]), _ptr(k.tiles["blob"]), B.shape[0], B.shape[1],
+                                         _ptr(k.tile_bound), _ptr(k.perm_b), k.tiles["stage_bytes"], _ptr(row_buf),
+                                         _ptr(col_buf), capacity, k.counter(0), k.counter(1), k.counter(2), p.warps,
+                                         _stream()))
         LAUNCH_COUNTS["tiles"] += 3
+        return
+    k.counters.zero_()
+    _lib.check(L.sg_cossim_candidates(
+        _ptr(A.d_indptr), _ptr(l_len), _ptr(l_idx), _ptr(l_val), k.row_begin, k.row_begin + n, _ptr(perm),
+        B.shape[0], A.shape[1], _ptr(k.bucket_dir), _ptr(k.bucket_maxw), _ptr(k.post), _ptr(k.perm_b), p.tile_w,
+        _lib.SG_ACC_U16 if p.acc == "u16" else _lib.SG_ACC_F32, max(B.norm_bound, 1.0),
+        p.thr_c, _ptr(l_thr), _ptr(l_xp), _ptr(k.tile_bound), p.tiles_per_group, _ptr(row_buf), _ptr(col_buf),
+        _ptr(partial_buf), capacity, k.counter(0), k.counter(1), p.warps, _stream()))
+    LAUNCH_COUNTS["candidates"] += 1
 
-    def launch(perm, rb, re_, row_buf, col_buf, capacity, partial_buf=None):
-        if use_tiles:
-            return launch_tiles(perm, re_ - rb, row_buf, col_buf, capacity)
-        l_idx, l_val, l_len, l_thr, l_xp, _ = pruned["arrays"]
-        counters.zero_()
-        _lib.check(L.sg_cossim_candidates(
-            _ptr(A.d_indptr), _ptr(l_len), _ptr(l_idx), _ptr(l_val), rb, re_, _ptr(perm), n_right,
-            A.shape[1], _ptr(bucket_dir), _ptr(bucket_maxw), _ptr(post), _ptr(perm_b), tile_w, acc_code,
-            max(B.norm_bound, 1.0),
-            thr_c, _ptr(l_thr), _ptr(l_xp), _ptr(tile_bound), tiles_per_group, _ptr(row_buf), _ptr(col_buf),
-            _ptr(partial_buf), capacity, c_count, c_queue, warps, _stream()))
-        LAUNCH_COUNTS["candidates"] += 1
 
-    # Exact threshold pruning of the left rows (the fixed-point tile always takes per-row thresholds: its margin
-    # grows with the number of features added).  A counting pass over a sample of the rows (in processing order,
-    # so clusters of identical names are sampled in proportion) sizes the candidate buffers; when the caller left
-    # the pruning level open and the sample reports more than MAX_CAND_DENSITY candidates per (row, column) pair,
-    # the level is lowered: every candidate costs an exact re-score, every skipped posting saves one update.
-    levels = [prune]
-    if prune_auto and prune > 0.0 and thr_c > 0.0:
-        levels = [prune, 0.75 * prune, 0.5 * prune, 0.25 * prune, 0.0]
+def _cand_buffers(k, capacity):
+    """(rows, columns, partial scores | None) of `capacity` candidates."""
+    t = torch()
+    dev = k.A.device
+    return (_empty(capacity, t.int32, dev), _empty(capacity, t.int32, dev),
+            _empty(capacity, t.float32, dev) if k.plan.refine else None)
 
-    def prepare(level):
-        if (level > 0.0 and thr_c > 0.0) or margin_pf > 0.0:
-            pruned["arrays"] = prune_left(A, B, hrank, row_begin, row_end, float(threshold), margin, margin_pf,
-                                          level if thr_c > 0.0 else 0.0)
-        else:
-            pruned["arrays"] = (A.d_indices, A.d_val32, None, None, None, None)
 
-    def timed_launch(perm, rb, re_, row_buf, col_buf, capacity, partial_buf=None):
-        if _timed(stats):
-            ev0, ev1 = t.cuda.Event(enable_timing=True), t.cuda.Event(enable_timing=True)
-            ev0.record()
-        launch(perm, rb, re_, row_buf, col_buf, capacity, partial_buf)
-        if _timed(stats):
-            ev1.record()
-            stats.setdefault("candidate_events", []).append((ev0, ev1))
-        head = counters[:4].cpu().numpy()
-        if use_tiles and stats is not None:
-            stats["pairs_walked"] = stats.get("pairs_walked", 0) + int(head[2])
-            stats["postings_walked"] = stats.get("postings_walked", 0) + int(head[3])
-        return int(head[0])
+def _timed_candidates(k, pruned, perm, n, bufs, capacity, stats):
+    """A candidates launch that produces candidates (sizing passes do not): timed for bench.py's kernel time, the
+    walk counters of the tile kernel added to stats.  Returns the number of candidates."""
+    t = torch()
+    if _timed(stats):
+        ev0, ev1 = t.cuda.Event(enable_timing=True), t.cuda.Event(enable_timing=True)
+        ev0.record()
+    _launch_candidates(k, pruned, perm, n, bufs[0], bufs[1], capacity, bufs[2])
+    if _timed(stats):
+        ev1.record()
+        stats.setdefault("candidate_events", []).append((ev0, ev1))
+    head = k.counters[:4].cpu().numpy()
+    if k.plan.kernel == "tiles" and stats is not None:
+        stats["pairs_walked"] = stats.get("pairs_walked", 0) + int(head[2])
+        stats["postings_walked"] = stats.get("postings_walked", 0) + int(head[3])
+    return int(head[0])
 
-    fixed_cap = bool(os.environ.get("SG_B200_CAND_CAP"))
-    sample = None
-    if not fixed_cap and n_rows >= 65536:
-        stride = max(64, n_rows // 8192)
-        sample = perm_a[:n_rows:stride].contiguous()
-    est = None
-    first = None          # (cand_row, cand_col, n_cand) of a whole-range launch that needed no sizing pass
-    search = True
-    dense = MAX_CAND_DENSITY * n_rows * n_right
-    # The sizing pass is latency-bound (a few thousand rows against every column tile, cold: 2-3 ms whatever the
-    # shard).  While a wasted launch costs no more than a few tens of ms, launch everything at once at the first
-    # level into buffers of the density limit; only an overflow or a count above the limit falls back to the
-    # sample / level search / row chunks below, and then the exact count of the first level is already known.
-    # Candidates of the fixed-point row kernel carry their partial score: sg_rescore_refined re-tests each with the
-    # grouped bound (csrc/sg_prune.cu) before its right row is read.
-    refine = REFINE and not use_tiles and acc == "u16" and margin_pf > 0.0
-    if not fixed_cap and float(n_rows) * float(n_right) <= OPTIMISTIC_PAIRS:
-        prune = levels[0]
-        prepare(prune)
-        cap0 = int(min(int(dense) + (1 << 22), CAND_CHUNK))
-        cand_row0 = _empty(cap0, t.int32, dev)
-        cand_col0 = _empty(cap0, t.int32, dev)
-        cand_part0 = _empty(cap0, t.float32, dev) if refine else None
+
+def _size_candidates(k, stats):
+    """Pruning level and candidate buffers of the call: (level, pruned rows at that level, candidate estimate | None,
+    (rows, columns, partial scores, count) of a whole-range launch that already holds every candidate | None).
+
+    Every candidate costs an exact re-score and every skipped posting saves one update, so with several levels
+    (plan.levels) the level is lowered while the candidates exceed plan.cand_limit.  Three strategies:
+      1. whole range (plan.whole_range): a sizing pass is latency-bound (a few thousand rows against every column
+         tile, cold: 2-3 ms whatever the shard) while a wasted launch over a moderate range costs no more than a few
+         tens of ms.  So all rows are launched at the first level into buffers of the density limit.  When their
+         candidates fit and are not too many, that is the answer; when they overflow the buffers without exceeding the
+         limit, the exact count is the estimate at this level; when they exceed the limit, the sample search below
+         goes on from the next level.
+      2. sample (plan.sample_stride): a counting pass over every stride-th row of the processing order (clusters of
+         identical names are sampled in proportion) per level, down the levels until the estimate is within the limit.
+      3. neither: the first level and no estimate; the chunk loop sizes its buffer from the row count."""
+    p = k.plan
+    levels = p.levels
+    sample = k.perm_a[:k.n_rows:p.sample_stride].contiguous() if p.sample_stride else None
+    dummy = _empty(1, torch().int32, k.A.device)          # the counting pass stores no candidate
+    if p.whole_range:
+        pruned = _prune(k, levels[0])
+        capacity = int(min(int(p.cand_limit) + (1 << 22), CAND_CHUNK))
+        bufs = _cand_buffers(k, capacity)
         mark(stats, "prune_sample")
-        n0 = timed_launch(perm_a, row_begin, row_end, cand_row0, cand_col0, cap0, cand_part0)
+        n = _timed_candidates(k, pruned, k.perm_a, k.n_rows, bufs, capacity, stats)
         mark(stats, "candidates")
-        too_dense = len(levels) > 1 and sample is not None and n0 > dense
-        if n0 <= cap0 and not too_dense:
-            first = (cand_row0, cand_col0, cand_part0, n0)
-            search = False
-        else:
-            del cand_row0, cand_col0, cand_part0
-            if _timed(stats):
-                stats["wasted_launch"] = True
-            if too_dense:
-                levels = levels[1:]
-            else:
-                est, search = n0, False          # stay at this level: chunks / buffers from the exact count
-    if search:
-        for level in levels:
-            prepare(level)
-            prune = level
-            if sample is None:
-                break
-            launch(sample, row_begin, row_begin + int(sample.numel()), dummy, dummy, 0)
-            est = int(counters[0].item()) * stride
-            if est <= dense:
-                break
-    l_idx, l_val, l_len, l_thr, l_xp, l_xg = pruned["arrays"]
+        too_dense = len(levels) > 1 and sample is not None and n > p.cand_limit
+        if n <= capacity and not too_dense:
+            return levels[0], pruned, None, bufs + (n,)
+        del bufs
+        if _timed(stats):
+            stats["wasted_launch"] = True
+        if not too_dense:
+            return levels[0], pruned, n, None
+        levels = levels[1:]
+    est = None
+    for level in levels:
+        pruned = _prune(k, level)
+        if sample is None:
+            break
+        _launch_candidates(k, pruned, sample, int(sample.numel()), dummy, dummy, 0)
+        est = int(k.counters[0].item()) * p.sample_stride
+        if est <= p.cand_limit:
+            break
+    return level, pruned, est, None
+
+
+def _count_macs(k, pruned):
+    """(postings of B the kept features of the pruned left rows walk, kept features): stats["count_macs"]."""
+    t = torch()
+    A, n_left = k.A, k.A.shape[0]
+    l_idx, _, l_len = pruned[:3]
+    df = feature_df(k.B).long()
+    pos = t.arange(A.d_indices.numel(), device=A.device)
+    rid = t.searchsorted(A.d_indptr[:n_left + 1].contiguous(), pos, right=True) - 1
+    ok = (rid >= k.row_begin) & (rid < k.row_end)
+    rid = rid.clamp(0, n_left - 1)
+    live = ok & ((pos - A.d_indptr[rid]) < l_len[rid].long())
+    return int(df[l_idx.long().clamp(0, A.shape[1] - 1)][live].sum().item()), int(live.sum().item())
+
+
+def _chunk_candidates(k, pruned, perm, n, capacity, stats):
+    """(rows, columns, partial scores, count) of the candidates of the left rows perm[:n]; buffers that overflow are
+    allocated again with the exact count."""
+    for attempt in range(3):
+        bufs = _cand_buffers(k, capacity)
+        n_cand = _timed_candidates(k, pruned, perm, n, bufs, capacity, stats)
+        if n_cand <= capacity:
+            return bufs + (n_cand,)
+        if n_cand * 24 > 96 * 2**30:
+            raise OverflowError("%d candidate pairs above the threshold do not fit the candidate buffer; "
+                                "raise min_similarity or split the input" % n_cand)
+        capacity = n_cand
+    raise OverflowError("candidate buffer overflow")
+
+
+def _rescore(k, pruned, cands, row_cnt, last, stats):
+    """Exact scores of one chunk's candidates; only the pairs strictly above the threshold are kept, and counted per
+    left row in row_cnt.  Returns (rows, columns, scores, kept count, survivors of the longest row when `last`)."""
+    t = torch()
+    L = _lib.load()
+    A, B, dev = k.A, k.B, k.A.device
+    cand_row, cand_col, cand_part, n_cand = cands
+    _, _, _, l_thr, _, l_xg = pruned
+    dt = _lib.SG_DTYPE_F32 if A.dtype == np.float32 else _lib.SG_DTYPE_F64
+    score = _empty(n_cand, t.float64, dev)
+    keep_row = _empty(n_cand, t.int32, dev)
+    keep_col = _empty(n_cand, t.int32, dev)
+    k.counters.zero_()
+    if k.plan.refine:
+        _lib.check(L.sg_rescore_refined(n_cand, _ptr(cand_row), _ptr(cand_col), _ptr(cand_part), _ptr(l_xg),
+                                        _ptr(B._heavy_groups), _ptr(l_thr), _ptr(A.d_indptr), _ptr(A.d_indices),
+                                        _ptr(A.d_val), _ptr(B.d_indptr), _ptr(B.d_indices), _ptr(B.d_val), dt,
+                                        _ptr(score), k.threshold, _ptr(keep_row), _ptr(keep_col), k.counter(0),
+                                        k.counter(2), _ptr(row_cnt), k.row_begin, _stream()))
+    else:
+        _lib.check(L.sg_rescore(n_cand, _ptr(cand_row), _ptr(cand_col), _ptr(A.d_indptr), _ptr(A.d_indices),
+                                _ptr(A.d_val), _ptr(B.d_indptr), _ptr(B.d_indices), _ptr(B.d_val), dt,
+                                _ptr(score), k.threshold, _ptr(keep_row), _ptr(keep_col), k.counter(0),
+                                _ptr(row_cnt), k.row_begin, _stream()))
+    LAUNCH_COUNTS["rescore"] += 1
+    if last:      # the largest row rides along with the read-back
+        _lib.check(L.sg_row_count_max(k.n_rows, _ptr(row_cnt), k.counter(1), _stream()))
+    head = k.counters[:3].cpu().numpy()
+    if k.plan.refine and stats is not None:
+        stats["n_refined"] = stats.get("n_refined", 0) + int(head[2])
+    return keep_row, keep_col, score, int(head[0]), int(head[1])
+
+
+def _candidates_rescored(k, stats):
+    """Pruning level and sizing (_size_candidates), then the candidates of the left rows chunk by chunk (slices of the
+    processing order), each chunk re-scored exactly right away.  Returns the survivors (rows, columns, scores, count),
+    their count per left row and that of the longest row."""
+    t = torch()
+    dev, n_rows = k.A.device, k.n_rows
+    # sized here so that only the chunk loop holds the whole-range launch's buffers (released after their re-score)
+    level, pruned, est, first = _size_candidates(k, stats)
     mark(stats, "prune_sample")
     if stats is not None:
-        stats["prune"], stats["acc"] = prune, acc
-        stats["kernel"] = "tiles" if use_tiles else "row"
+        stats["prune"], stats["acc"] = level, k.plan.acc
+        stats["kernel"] = k.plan.kernel
         stats["n_candidates_estimate"] = est
-        if stats.get("count_macs") and l_len is not None:
-            df = feature_df(B).long()
-            pos = t.arange(A.d_indices.numel(), device=dev)
-            rid = t.searchsorted(A.d_indptr[:n_left + 1].contiguous(), pos, right=True) - 1
-            ok = (rid >= row_begin) & (rid < row_end)
-            rid = rid.clamp(0, n_left - 1)
-            live = ok & ((pos - A.d_indptr[rid]) < l_len[rid].long())
-            stats["macs_walked"] = int(df[l_idx.long().clamp(0, A.shape[1] - 1)][live].sum().item())
-            stats["features_kept"] = int(live.sum().item())
-
-    # Left rows are taken in chunks (slices of the processing order) whose candidates fit CAND_CHUNK entries;
-    # every chunk is re-scored exactly right away and only the pairs strictly above the threshold are kept.
-    n_chunks = 1 if est is None else max(1, -(-int(1.3 * est) // CAND_CHUNK))
-    rows_per_chunk = -(-n_rows // n_chunks)
+        if stats.get("count_macs") and pruned[2] is not None:
+            stats["macs_walked"], stats["features_kept"] = _count_macs(k, pruned)
+    n_chunks, rows_per_chunk = row_chunks(n_rows, est)
     kept = []
     n_cand_total = 0
-    max_row_cnt = 0
     row_cnt = t.zeros(n_rows + 1, dtype=t.int32, device=dev)      # survivors per left row (sg_rescore)
     for lo in range(0, n_rows, rows_per_chunk):
         hi = min(lo + rows_per_chunk, n_rows)
-        perm_chunk = perm_a if (lo == 0 and hi == n_rows) else perm_a[lo:hi]
-        if est is not None:
-            cap = min(max(int(1.3 * est * (hi - lo) / n_rows) + (1 << 22), 1 << 22), 1 << 31)
-        for attempt in range(3):
-            if first is not None:
-                cand_row, cand_col, cand_part, n_cand = first
-                first = None
-                break
-            cand_row = _empty(cap, t.int32, dev)
-            cand_col = _empty(cap, t.int32, dev)
-            cand_part = _empty(cap, t.float32, dev) if refine else None
-            n_cand = timed_launch(perm_chunk, row_begin, row_begin + (hi - lo), cand_row, cand_col, cap, cand_part)
-            if n_cand <= cap:
-                break
-            if n_cand * 24 > 96 * 2**30:
-                raise OverflowError("%d candidate pairs above the threshold do not fit the candidate buffer; "
-                                    "raise min_similarity or split the input" % n_cand)
-            cap = n_cand
+        if first is not None:        # only without an estimate, i.e. in one chunk
+            cands, first = first, None
         else:
-            raise OverflowError("candidate buffer overflow")
-        n_cand_total += n_cand
+            perm = k.perm_a if (lo == 0 and hi == n_rows) else k.perm_a[lo:hi]
+            cands = _chunk_candidates(k, pruned, perm, hi - lo, chunk_capacity(n_rows, hi - lo, est), stats)
+        n_cand_total += cands[3]
         mark(stats, "candidates")
-        # exact scores; only the candidates strictly above the threshold go on to the selection sorts
-        score = _empty(n_cand, t.float64, dev)
-        keep_row = _empty(n_cand, t.int32, dev)
-        keep_col = _empty(n_cand, t.int32, dev)
-        counters.zero_()
-        if refine and cand_part is not None and l_xg is not None:
-            _lib.check(L.sg_rescore_refined(n_cand, _ptr(cand_row), _ptr(cand_col), _ptr(cand_part), _ptr(l_xg),
-                                            _ptr(B._heavy_groups), _ptr(l_thr), _ptr(A.d_indptr), _ptr(A.d_indices),
-                                            _ptr(A.d_val), _ptr(B.d_indptr), _ptr(B.d_indices), _ptr(B.d_val), dt,
-                                            _ptr(score), float(threshold), _ptr(keep_row), _ptr(keep_col), c_count,
-                                            c_walk, _ptr(row_cnt), row_begin, _stream()))
-        else:
-            _lib.check(L.sg_rescore(n_cand, _ptr(cand_row), _ptr(cand_col), _ptr(A.d_indptr), _ptr(A.d_indices),
-                                    _ptr(A.d_val), _ptr(B.d_indptr), _ptr(B.d_indices), _ptr(B.d_val), dt,
-                                    _ptr(score), float(threshold), _ptr(keep_row), _ptr(keep_col), c_count,
-                                    _ptr(row_cnt), row_begin, _stream()))
-        LAUNCH_COUNTS["rescore"] += 1
-        if lo + rows_per_chunk >= n_rows:      # last chunk: the largest row rides along with the read-back
-            _lib.check(L.sg_row_count_max(n_rows, _ptr(row_cnt), c_queue, _stream()))      # counters[1], zeroed above
-        head = counters[:3].cpu().numpy()
-        n_keep, max_row_cnt = int(head[0]), int(head[1])
-        if refine and stats is not None:
-            stats["n_refined"] = stats.get("n_refined", 0) + int(head[2])
+        keep_row, keep_col, score, n_keep, max_row_cnt = _rescore(k, pruned, cands, row_cnt, hi == n_rows, stats)
         mark(stats, "rescore")
         if n_chunks > 1:      # release the chunk-sized buffers, keep the survivors
             keep_row, keep_col, score = keep_row[:n_keep].clone(), keep_col[:n_keep].clone(), score[:n_keep].clone()
         kept.append((keep_row, keep_col, score, n_keep))
-        del cand_row, cand_col, cand_part
+        del cands
     if len(kept) == 1:
         cand_row, cand_col, score, n_cand = kept[0]
     else:
-        n_cand = sum(k[3] for k in kept)
-        cand_row = t.cat([k[0][:k[3]] for k in kept]) if n_cand else _empty(1, t.int32, dev)
-        cand_col = t.cat([k[1][:k[3]] for k in kept]) if n_cand else _empty(1, t.int32, dev)
-        score = t.cat([k[2][:k[3]] for k in kept]) if n_cand else _empty(1, t.float64, dev)
-    del kept
+        n_cand = sum(x[3] for x in kept)
+        cand_row = t.cat([x[0][:x[3]] for x in kept]) if n_cand else _empty(1, t.int32, dev)
+        cand_col = t.cat([x[1][:x[3]] for x in kept]) if n_cand else _empty(1, t.int32, dev)
+        score = t.cat([x[2][:x[3]] for x in kept]) if n_cand else _empty(1, t.float64, dev)
     if stats is not None:
         stats["n_candidates"] = n_cand_total
         stats["n_above_threshold"] = n_cand
         stats["n_row_chunks"] = n_chunks
-        stats["tile_w"], stats["warps"], stats["n_tiles"] = tile_w, warps, T
-        stats["tiles_per_group"] = tiles_per_group
-        if use_tiles:
-            stats["stage_bytes"] = tiles["stage_bytes"]
+    return cand_row, cand_col, score, n_cand, row_cnt, max_row_cnt
 
+
+def _select(k, top_n, cand_row, cand_col, score, n_cand, row_cnt, max_row_cnt, stats):
+    """The top_n survivors of every left row, by descending score (one read-back: match count and longest row)."""
+    t = torch()
+    L = _lib.load()
+    dev, n_rows, row_begin = k.A.device, k.n_rows, k.row_begin
     out_indptr = _empty(n_rows + 1, t.int64, dev)
     out_row = _empty(n_cand, t.int32, dev)
     out_col = _empty(n_cand, t.int32, dev)
     out_score = _empty(n_cand, t.float64, dev)
     tail = t.zeros(2, dtype=t.int64, device=dev)            # [0] out_nnz, [1] max_row (int32 view)
-    rows_cap = int(L.sg_topn_rows_cap())
-    if (top_n <= 32 or max_row_cnt <= rows_cap or top_n <= rows_cap // 2) and SELECT_MODE != "sort":
-        # survivors bucketed by row, every row ranked on its own (warp shuffle network / one CTA in shared memory)
+    c_nnz, c_max = ctypes.c_void_p(tail.data_ptr()), ctypes.c_void_p(tail.data_ptr() + 8)
+    mode = select_mode(top_n, max_row_cnt, int(L.sg_topn_rows_cap()))
+    if mode == "rows":
         ws_bytes = int(L.sg_topn_select_rows_workspace_bytes(n_cand, n_rows))
         ws = _empty(ws_bytes, t.uint8, dev)
         _lib.check(L.sg_topn_select_rows(n_cand, _ptr(cand_row), _ptr(cand_col), _ptr(score), row_begin, n_rows, top_n,
                                          _ptr(row_cnt), _ptr(out_indptr), _ptr(out_row), _ptr(out_col),
-                                         _ptr(out_score), ctypes.c_void_p(tail.data_ptr()),
-                                         ctypes.c_void_p(tail.data_ptr() + 8), _ptr(ws), ws_bytes, _stream()))
+                                         _ptr(out_score), c_nnz, c_max, _ptr(ws), ws_bytes, _stream()))
         LAUNCH_COUNTS["select"] += 6
-        if stats is not None:
-            stats["select"] = "rows"
     else:
-        # a row with more survivors than one CTA ranks in shared memory: three global radix sorts
         ws_bytes = int(L.sg_topn_select_workspace_bytes(n_cand, n_rows))
         ws = _empty(ws_bytes, t.uint8, dev)
         _lib.check(L.sg_topn_select(n_cand, _ptr(cand_row), _ptr(cand_col), _ptr(score), row_begin, n_rows, top_n,
-                                    float(threshold), _ptr(out_indptr), _ptr(out_row), _ptr(out_col), _ptr(out_score),
-                                    ctypes.c_void_p(tail.data_ptr()), ctypes.c_void_p(tail.data_ptr() + 8), _ptr(ws),
-                                    ws_bytes, _stream()))
+                                    k.threshold, _ptr(out_indptr), _ptr(out_row), _ptr(out_col), _ptr(out_score),
+                                    c_nnz, c_max, _ptr(ws), ws_bytes, _stream()))
         LAUNCH_COUNTS["select"] += 7
-        if stats is not None:
-            stats["select"] = "sort"
+    if stats is not None:
+        stats["select"] = mode
     th = tail.cpu().numpy()
     mark(stats, "select")
-    nnz = int(th[0])
-    max_row = int(th[1:2].view(np.int32)[0])
-    return DeviceMatches(shape, out_row, out_col, out_score, nnz, max_row, indptr=out_indptr)
+    return DeviceMatches((k.A.shape[0], k.B.shape[0]), out_row, out_col, out_score, int(th[0]),
+                         int(th[1:2].view(np.int32)[0]), indptr=out_indptr)
 
 
 def symmetrize(M, fix_diagonal=True, mirror=True):
